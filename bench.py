@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json metric: audio frames/sec (22.05 kHz) of the generator forward.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one generator forward over one synthetic batch of config 2 (B=64 mel segments of
 80 x 32 frames -> 64 x 8192 audio frames) per GPU.  1 audio frame = 1 PCM sample; 1 mel frame = 256
@@ -18,6 +18,9 @@ audio frames (SURVEY 8d).  Weights are seeded random-init (melgan_multi_b200.syn
              number of iterations, median; rank 0 at N=1 only.
   --impl reference   times that same CPU port as the reference arm at the same config (the reference is pure
              Python and /root/reference does not exist on the GPU box); value from the MEDIAN step.
+  --dump-outputs DIR   writes what the timed path returned in its last timed step, rank 0's [64, 1, 8192] fp32 audio
+             (2 MB), to DIR/audio.npy.  Weights and mel inputs are seeded, so runs with the same arguments see the
+             same inputs and two builds can be compared output for output.
 """
 import argparse
 import ctypes
@@ -370,7 +373,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--cpu-budget", type=float, default=15.0, help="seconds of CPU-baseline timing")
     ap.add_argument("--no-multi", action="store_true", help="skip the DDP train-step / utterance-shard blocks at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the audio of the last timed step (rank 0) to DIR/audio.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of the b200 path")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -430,6 +439,8 @@ def main():
         gd.forward(mels[k % 4], out)
         ev[k][1].record()
     barrier()
+    # the passes below reuse `out`: keep the last timed step's result now
+    last_audio = out.cpu().numpy() if args.dump_outputs and rank == 0 else None
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = max_over_ranks(sum(step_ms))
     frames_per_step = B * T * 256 * world
@@ -550,6 +561,9 @@ def main():
 
     multi = multi_gpu_blocks(dev, rank, world, barrier, max_over_ranks) if world > 1 and not args.no_multi else None
 
+    if last_audio is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "audio.npy"), last_audio)
     if rank == 0:
         emit(({
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,

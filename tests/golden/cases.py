@@ -19,6 +19,21 @@ def gen_key(B, T, seed, realistic):
     return "gen_B%d_T%d_s%d_r%d" % (B, T, seed, int(realistic))
 
 
+CONFIG2_SAMPLES = 1024  # of each item's 8192 output samples kept in config2_outputs.npz (keeps the file under 1 MB)
+CONFIG2_BLOCK = 64      # samples per float64 block sum; the block sums cover every sample
+
+
+def config2_sample_index():
+    return np.sort(np.random.RandomState(8192).choice(8192, CONFIG2_SAMPLES, replace=False))
+
+
+def config2_digest(y, index):
+    """What config2_outputs.npz keeps of a [B, 1, 8192] generator output: the samples at `index` (the same positions in
+    every item) and the float64 sums of every block of CONFIG2_BLOCK consecutive samples."""
+    y = np.asarray(y).reshape(len(y), -1)
+    return y[:, index], y.astype(np.float64).reshape(len(y), -1, CONFIG2_BLOCK).sum(axis=2)
+
+
 def op_inputs():
     """Yields (key, kind, params, x, w, b) in a fixed draw order from RandomState(99)."""
     rs = np.random.RandomState(99)

@@ -1,9 +1,8 @@
 """Generate the golden fixtures in tests/golden/ by running the UNMODIFIED reference.
 
-Run in the build container only (it imports /root/reference/models.py, which does not exist
-on the GPU box):
+It imports models.py from a checkout of the reference, named by MG_REFERENCE_DIR:
 
-    python tests/golden/make_golden.py
+    MG_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden.py
 
 Weights come from melgan_multi_b200.synth (seeded numpy MT19937), loaded into the reference
 modules through load_state_dict, so the fixtures hold inputs' seeds and the reference's
@@ -19,7 +18,10 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+REFERENCE = os.environ.get("MG_REFERENCE_DIR", "")
+if not os.path.isfile(os.path.join(REFERENCE, "models.py")):
+    raise SystemExit("set MG_REFERENCE_DIR to the reference checkout (the directory holding its models.py)")
+sys.path.insert(0, REFERENCE)
 warnings.filterwarnings("ignore")
 
 import models as ref_models  # noqa: E402  (the reference)
@@ -67,13 +69,18 @@ TRAIN_CASE_B16 = dict(B=16, T=32, mel_seed=0, audio_seed=0)  # BASELINE config 3
 
 def config2_golden():
     """BASELINE config 2 at full size (B=64, 80x32 mel -> 64x8192 samples) through the unmodified reference on CPU, for
-    N(0,1) and log-mel-like inputs (2 x 2 MB): every item of the bench workload is pinned, not just item 0."""
+    N(0,1) and log-mel-like inputs: every item of the bench workload is pinned, not just item 0.  Of each output the
+    fixture keeps cases.config2_digest (a seeded sample of every item, block sums over every sample) and max |y|."""
     gen = load_state(ref_models.Generator(), synth.generator_state(1234))
-    out = {}
+    index = cases.config2_sample_index()
+    out = {"sample_index": index}
     with torch.no_grad():
         for realistic in (False, True):
             x = synth.mel_input(64, 32, 0, realistic)
-            out["gen_B64_T32_s0_r%d" % int(realistic)] = gen(torch.from_numpy(x)).numpy()
+            y = gen(torch.from_numpy(x)).numpy()
+            key = "gen_B64_T32_s0_r%d" % int(realistic)
+            out[key + "_sample"], out[key + "_blocksum"] = cases.config2_digest(y, index)
+            out[key + "_absmax"] = np.abs(y).max()
     path = os.path.join(HERE, "config2_outputs.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, "%.2f MB" % (os.path.getsize(path) / 1e6), len(out), "arrays")
@@ -148,7 +155,10 @@ def main():
         out["gen_T1000_tail"] = y[-4096:].copy()
         out["gen_T1000_blocksum"] = y.astype(np.float64).reshape(250, 1024).sum(axis=1)
         # weight-norm fold as the reference modules apply it (pre-forward hook output)
-        out["fold_conv_pre"] = gen.conv_pre.weight.detach().numpy()
+        # conv_pre's fold is 1.1 MB: keep every 8th output channel, and the L2 norm of every channel
+        fold = gen.conv_pre.weight.detach().numpy()
+        out["fold_conv_pre_every8th"] = fold[::8].copy()
+        out["fold_conv_pre_norms"] = np.sqrt((fold.astype(np.float64) ** 2).reshape(len(fold), -1).sum(axis=1))
         out["fold_ups3"] = gen.ups[3].weight.detach().numpy()
         out["fold_res2_c1_1"] = gen.resblocks[2].convs1[1].weight.detach().numpy()
 

@@ -111,17 +111,21 @@ def config2_golden():
 @pytest.mark.parametrize("realistic", [False, True])
 def test_config2_full_size_matches_reference(host_engine, gen_module, config2_golden, realistic):
     """BASELINE config 2 at FULL size (B=64, 80x32 mel -> 64x8192 samples), every one of the 64 items against the
-    unmodified reference's CPU-fp32 output (tests/golden/config2_outputs.npz, written by make_golden.py --config2), for
-    N(0,1) and log-mel-like inputs, through both entry points (host buffers, torch module)."""
+    unmodified reference's CPU-fp32 output (tests/golden/config2_outputs.npz, written by make_golden.py --config2: a
+    seeded sample of every item and block sums over every sample), for N(0,1) and log-mel-like inputs, through both
+    entry points (host buffers, torch module)."""
     x = synth.mel_input(64, 32, 0, realistic)
-    ref = config2_golden["gen_B64_T32_s0_r%d" % int(realistic)]
+    key = "gen_B64_T32_s0_r%d" % int(realistic)
+    ref, ref_bsum = config2_golden[key + "_sample"], config2_golden[key + "_blocksum"]
     y = host_engine.forward(x)
-    assert y.shape == ref.shape == (64, 1, 8192)
-    scale = np.abs(ref).max()
-    per_item = np.abs(y.astype(np.float64) - ref).reshape(64, -1).max(axis=1) / scale
+    assert y.shape == (64, 1, 8192)
+    ys, bsum = cases.config2_digest(y, config2_golden["sample_index"])
+    scale = float(config2_golden[key + "_absmax"])
+    per_item = np.abs(ys.astype(np.float64) - ref).max(axis=1) / scale
     assert per_item.max() <= TOL, (int(per_item.argmax()), float(per_item.max()))
-    m, l2 = rel_errors(y, ref)
+    m, l2 = rel_errors(ys, ref)
     assert m <= TOL and l2 <= TOL, (m, l2)
+    assert np.abs(bsum - ref_bsum).max() <= cases.CONFIG2_BLOCK * TOL * scale
     with torch.no_grad():
         yd = gen_module(torch.from_numpy(x).cuda()).cpu().numpy()
     assert np.array_equal(yd, y)
