@@ -77,6 +77,19 @@ size_t mg_gen_workspace_bytes(int B, int T);
 int mg_gen_forward(const void *packed, const float *mel, float *audio, int B, int T,
                    void *workspace, size_t workspace_bytes, void *stream);
 
+/* Ragged batch: mel [B, 80, T] padded, item b is its first lengths[b] frames (lengths: HOST array of B ints, each in
+ * [1, T]).  audio [B, 1, 256*T]: audio[b, :, :256*lengths[b]] equals the forward of mel[b:b+1, :, :lengths[b]] alone, bit for
+ * bit, and audio[b, :, 256*lengths[b]:] is exactly 0.  The padding frames of mel are never read (NaN there changes
+ * nothing) and no result depends on earlier workspace contents.  workspace: mg_gen_workspace_bytes(B, T) bytes, as for
+ * the uniform call; mg_gen_check_status(workspace, B, T, stream) reports on it.  Asynchronous on `stream` (no host
+ * synchronisation, no allocation, no host-to-device copy: the per-item tables are kernel parameters), so the call can be
+ * captured in a CUDA graph.  Only the frames that exist are computed: the batch slices are cut by cumulative frames.
+ * Always runs the default kernel chain: mg_gen_set_pipeline / MG_GEN_TAIL (A/B knobs of the uniform call) do not apply.
+ * Invalid arguments (lengths NULL, or a lengths[i] outside [1, T]) return MG_ERR_INVALID_ARGUMENT before any CUDA call;
+ * the message names the index. */
+int mg_gen_forward_varlen(const void *packed, const float *mel, float *audio, int B, int T, const int *lengths,
+                          void *workspace, size_t workspace_bytes, void *stream);
+
 /* Same as mg_gen_forward, but brackets each of the mg_gen_forward_launches() kernels with CUDA
  * events on `stream`, waits for the last one and returns the per-kernel device times in
  * kernel_ms[0 .. mg_gen_forward_launches()-1] (names: mg_gen_kernel_name(i)).  Used by bench.py for the
@@ -184,6 +197,9 @@ int mg_gen_engine_load_state(mg_gen_engine *e, const float *const *v, const floa
  * buffer.  The copies are cut with the batch slices (mg_gen_forward_slices): a slice's audio goes
  * back to the host while the other slices are still computing. */
 int mg_gen_engine_forward(mg_gen_engine *e, const float *mel_host, float *audio_host, int B, int T);
+/* The ragged form (contract of mg_gen_forward_varlen; lengths: HOST array of B ints in [1, T]): mel_host [B,80,T] padded,
+ * audio_host [B,1,256T] with exact zeros past each item's 256*lengths[b] samples.  Synchronous, like mg_gen_engine_forward. */
+int mg_gen_engine_forward_varlen(mg_gen_engine *e, const float *mel_host, float *audio_host, int B, int T, const int *lengths);
 /* Device time of the last forward in milliseconds (CUDA events on the engine's stream around the sliced
  * upload -> kernels -> download sequence). */
 int mg_gen_engine_last_kernel_ms(mg_gen_engine *e, float *ms);

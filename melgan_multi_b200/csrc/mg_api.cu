@@ -15,11 +15,20 @@ static int *status_ptr(void *workspace, int B, int T) {
 }
 
 // mel_host / audio_host: optional pinned host buffers (the engine entry point); the copies ride on the batch slices' streams
+// lengths: optional host array of per-item lengths (ragged batch), already validated
 static int run_generator(const float *packed, const float *mel, float *audio, int B, int T, float *ws, cudaStream_t s,
-                         cudaEvent_t *ev, const float *mel_host = nullptr, float *audio_host = nullptr) {
+                         cudaEvent_t *ev, const float *mel_host = nullptr, float *audio_host = nullptr, const int *lengths = nullptr) {
     int *st = status_ptr(ws, B, T);
     MG_CUDA_TRY(cudaMemsetAsync(st, 0, sizeof(int), s));
-    return launch_generator_tc(packed, mel, audio, B, T, ws, st, s, ev, mel_host, audio_host);
+    return launch_generator_tc(packed, mel, audio, B, T, ws, st, s, ev, mel_host, audio_host, lengths);
+}
+
+static int check_lengths(const char *fn, const int *lengths, int B, int T) {
+    if (!lengths) return set_error(MG_ERR_INVALID_ARGUMENT, "%s: lengths is NULL", fn);
+    for (int i = 0; i < B; ++i)
+        if (lengths[i] < 1 || lengths[i] > T)
+            return set_error(MG_ERR_INVALID_ARGUMENT, "%s: lengths[%d] = %d is outside [1, T = %d]", fn, i, lengths[i], T);
+    return MG_OK;
 }
 
 static int check_shape(const char *fn, int B, int T) {
@@ -91,6 +100,21 @@ int mg_gen_forward(const void *packed, const float *mel, float *audio, int B, in
     if ((uintptr_t)packed % 16 || (uintptr_t)workspace % 16)
         return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_forward: packed/workspace must be 16-byte aligned");
     return run_generator((const float *)packed, mel, audio, B, T, (float *)workspace, (cudaStream_t)stream, nullptr);
+}
+
+int mg_gen_forward_varlen(const void *packed, const float *mel, float *audio, int B, int T, const int *lengths, void *workspace,
+                          size_t workspace_bytes, void *stream) {
+    int rc = check_shape("mg_gen_forward_varlen", B, T);
+    if (rc) return rc;
+    if (!packed || !mel || !audio || !workspace) return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_forward_varlen: null argument");
+    if ((rc = check_lengths("mg_gen_forward_varlen", lengths, B, T))) return rc;
+    if (workspace_bytes < mg_gen_workspace_bytes(B, T))
+        return set_error(MG_ERR_WORKSPACE_TOO_SMALL, "mg_gen_forward_varlen: workspace %zu < %zu bytes", workspace_bytes,
+                         mg_gen_workspace_bytes(B, T));
+    if ((uintptr_t)packed % 16 || (uintptr_t)workspace % 16)
+        return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_forward_varlen: packed/workspace must be 16-byte aligned");
+    return run_generator((const float *)packed, mel, audio, B, T, (float *)workspace, (cudaStream_t)stream, nullptr, nullptr,
+                         nullptr, lengths);
 }
 
 int mg_gen_forward_timed(const void *packed, const float *mel, float *audio, int B, int T, void *workspace,
@@ -469,10 +493,8 @@ int mg_gen_engine_load_state(mg_gen_engine *e, const float *const *v, const floa
     return MG_OK;
 }
 
-int mg_gen_engine_forward(mg_gen_engine *e, const float *mel_host, float *audio_host, int B, int T) {
-    if (!e || !mel_host || !audio_host) return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_engine_forward: null argument");
-    int rc = check_shape("mg_gen_engine_forward", B, T);
-    if (rc) return rc;
+static int engine_forward(mg_gen_engine *e, const float *mel_host, float *audio_host, int B, int T, const int *lengths) {
+    int rc;
     if (!e->loaded) return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_engine_forward: no weights loaded");
     const size_t frames = (size_t)B * T;
     if ((rc = engine_reserve(e, frames))) return rc;
@@ -486,7 +508,7 @@ int mg_gen_engine_forward(mg_gen_engine *e, const float *mel_host, float *audio_
     if (!e->pin_status) MG_CUDA_TRY(cudaMallocHost(&e->pin_status, sizeof(int)));
     MG_CUDA_TRY(cudaEventRecord(e->ev0, e->stream));
     // upload, kernels and download are enqueued per batch slice (launch_generator_tc); one synchronisation at the end
-    rc = run_generator(e->packed, e->mel, e->audio, B, T, e->ws, e->stream, nullptr, src, out_pinned ? audio_host : e->pin_out);
+    rc = run_generator(e->packed, e->mel, e->audio, B, T, e->ws, e->stream, nullptr, src, out_pinned ? audio_host : e->pin_out, lengths);
     if (rc) return rc;
     MG_CUDA_TRY(cudaEventRecord(e->ev1, e->stream));
     *e->pin_status = 0;
@@ -497,6 +519,21 @@ int mg_gen_engine_forward(mg_gen_engine *e, const float *mel_host, float *audio_
         return set_error(MG_ERR_CUDA, "mg_gen_engine_forward: tensor-core pipeline wait timed out (code %d)", *e->pin_status);
     MG_CUDA_TRY(cudaEventElapsedTime(&e->last_ms, e->ev0, e->ev1));
     return MG_OK;
+}
+
+int mg_gen_engine_forward(mg_gen_engine *e, const float *mel_host, float *audio_host, int B, int T) {
+    if (!e || !mel_host || !audio_host) return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_engine_forward: null argument");
+    int rc = check_shape("mg_gen_engine_forward", B, T);
+    if (rc) return rc;
+    return engine_forward(e, mel_host, audio_host, B, T, nullptr);
+}
+
+int mg_gen_engine_forward_varlen(mg_gen_engine *e, const float *mel_host, float *audio_host, int B, int T, const int *lengths) {
+    if (!e || !mel_host || !audio_host) return set_error(MG_ERR_INVALID_ARGUMENT, "mg_gen_engine_forward_varlen: null argument");
+    int rc = check_shape("mg_gen_engine_forward_varlen", B, T);
+    if (rc) return rc;
+    if ((rc = check_lengths("mg_gen_engine_forward_varlen", lengths, B, T))) return rc;
+    return engine_forward(e, mel_host, audio_host, B, T, lengths);
 }
 
 int mg_gen_engine_last_kernel_ms(mg_gen_engine *e, float *ms) {

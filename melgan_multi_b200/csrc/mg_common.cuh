@@ -5,6 +5,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <type_traits>
+
 #include "../../include/melgan_b200.h"
 #include "mg_layout.h"
 
@@ -64,6 +66,43 @@ inline cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
+// Per-item mel lengths of one ragged generator launch (mg_gen_forward_varlen).  Passed BY VALUE as a __grid_constant__ kernel
+// parameter -- no device table, no copy, so the call stays asynchronous and graph-capturable.  Buffers keep the padded layout
+// [item][C][mul * T]; only the first mul * (cum[b+1] - cum[b]) positions of item b are sequence.
+//   cum[b]:   mel frames of the items before b (cum[n]: all of them)
+//   first[b]: ResBlock launches: grid.x index (in super-tiles) of item b's first tile, first[n] = super-tiles in all
+//   mul:      positions per mel frame at the kernel's input (1 conv_pre / up0, 8 res0, 64 res1, 64 up2, 128 res2, 256 res3)
+// kVlMaxItems bounds the items of one launch: the struct (2 KB) stays far below the 32 KB kernel-parameter limit (parameter
+// bytes are copied with every launch), and the launcher cuts a slice with more items into several launches.
+constexpr int kVlMaxItems = 256;
+struct VarLenTab {
+    int n, mul;
+    int cum[kVlMaxItems + 1];
+    int first[kVlMaxItems + 1];
+};
+struct NoVarLen {};  // the uniform instantiations' (empty) parameter in the same place
+template <bool VL>
+using VarLenArg = typename std::conditional<VL, VarLenTab, NoVarLen>::type;
+
+// the item that virtual row v (>= 0) belongs to when item b's rows start at  t.mul * t.cum[b] + pad * b;  t.n: past the last
+__device__ __forceinline__ int vl_item_of_row(const VarLenTab &t, int pad, int v) {
+    int lo = 0, hi = t.n;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (t.mul * t.cum[mid] + pad * mid <= v) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+// the item whose super-tiles [first[b], first[b+1]) contain grid index id (< first[n])
+__device__ __forceinline__ int vl_item_of_tile(const VarLenTab &t, int id) {
+    int lo = 0, hi = t.n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (t.first[mid] <= id) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
 // ---- launches implemented in the .cu files ------------------------------------------------
 int launch_pack(const float *const *v, const float *const *g, const float *const *bias, float *packed,
                 cudaStream_t s);
@@ -80,7 +119,13 @@ const char *generator_tc_kernel_config(int i, int T);
 const char *resblock_config_name(int stage, int L);
 int generator_tc_slices(int B, int T);  // batch slices (concurrent kernel chains) one forward is cut into
 int launch_generator_tc(const float *packed, const float *mel, float *audio, int B, int T, float *ws, int *status,
-                        cudaStream_t s, cudaEvent_t *ev = nullptr, const float *mel_host = nullptr, float *audio_host = nullptr);
+                        cudaStream_t s, cudaEvent_t *ev = nullptr, const float *mel_host = nullptr, float *audio_host = nullptr,
+                        const int *lengths = nullptr);
+int launch_gen_pre_tc_varlen(const float *mel, float *y, const float *packed, const VarLenTab &vt, int T, int *status, cudaStream_t s);
+int launch_convt_tc_varlen(const float *x, float *y, const float *packed, int stage, const VarLenTab &vt, int T, int *status,
+                           cudaStream_t s);
+int launch_resblock_tc_varlen(const float *x, float *y, const float *packed, int code, const VarLenTab &vt, int T, int *status,
+                              cudaStream_t s);
 int launch_gen_pre_tc(const float *mel, float *y, const float *packed, int B, int T, int *status, cudaStream_t s);
 int launch_disc_post1_tc(const float *x, float *y, const uint8_t *wtc, const float *bias, int Bt, int L, int *status,
                          cudaStream_t s);

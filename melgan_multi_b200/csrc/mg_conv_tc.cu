@@ -44,10 +44,12 @@ struct ConvCfg {
 
 // packed weights for this kernel: conv_tc_weight_index() in mg_layout.h
 
-template <class Cfg>
+// VL (generator conv_pre only): ragged batch -- item b's rows start at vl.cum[b] + PAD * b, its length is cum[b+1] - cum[b],
+// and L is the row stride of x / y (the padded length).  Uniform launches (VL = false) compile to the code without it.
+template <class Cfg, bool VL = false>
 __global__ void __launch_bounds__(Cfg::NT, Cfg::MINB)
 conv_rows_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const uint8_t *__restrict__ wtc,
-                    const float *__restrict__ bias, int L, int B, int *__restrict__ status) {
+                    const float *__restrict__ bias, int L, int B, int *__restrict__ status, const __grid_constant__ VarLenArg<VL> vl) {
     constexpr int CIN = Cfg::CIN, COUT = Cfg::COUT, NTAP = Cfg::NTAP, PAD = Cfg::PAD, KCA = Cfg::KCA, N = Cfg::N;
     constexpr int ROWS = Cfg::ROWS, APITCH = Cfg::APITCH, ASLOT = Cfg::ASLOT, BSLOT = Cfg::BSLOT;
     constexpr int NSA = Cfg::NSA, NSB = Cfg::NSB, NCONV = Cfg::NCONV;
@@ -145,8 +147,16 @@ conv_rows_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const ui
         bool ok = true;
         constexpr int NCH = CIN / KCA;
         const int v0 = r0 - PAD + tid;
-        const int item0 = v0 >= 0 ? v0 / Lv : 0, s0 = v0 - item0 * Lv;
-        const bool inr0 = (v0 >= 0 && item0 < B && s0 < L);
+        int item0, s0;
+        bool inr0;
+        if constexpr (VL) {
+            item0 = v0 >= 0 ? vl_item_of_row(vl, PAD, v0) : 0;
+            s0 = v0 - (vl.cum[item0] + PAD * item0);
+            inr0 = v0 >= 0 && item0 < vl.n && s0 < vl.cum[item0 + 1] - vl.cum[item0];
+        } else {
+            item0 = v0 >= 0 ? v0 / Lv : 0, s0 = v0 - item0 * Lv;
+            inr0 = (v0 >= 0 && item0 < B && s0 < L);
+        }
         const float *xrow = x + (size_t)(inr0 ? item0 : 0) * CIN * L + (inr0 ? s0 : 0);
         auto store_row = [&](uint8_t *slot, int i, const float *f) {
 #pragma unroll
@@ -162,8 +172,16 @@ conv_rows_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const ui
 #pragma unroll 1
             for (int i = NCONV + tid; i < ROWS + 2 * PAD; i += NCONV) {
                 const int v = r0 - PAD + i;
-                const int item = v >= 0 ? v / Lv : 0, s = v - item * Lv;
-                const bool inr = (v >= 0 && item < B && s < L);
+                int item, s;
+                bool inr;
+                if constexpr (VL) {
+                    item = v >= 0 ? vl_item_of_row(vl, PAD, v) : 0;
+                    s = v - (vl.cum[item] + PAD * item);
+                    inr = v >= 0 && item < vl.n && s < vl.cum[item + 1] - vl.cum[item];
+                } else {
+                    item = v >= 0 ? v / Lv : 0, s = v - item * Lv;
+                    inr = (v >= 0 && item < B && s < L);
+                }
                 const float *xp = x + ((size_t)(inr ? item : 0) * CIN + ca * KCA) * L + (inr ? s : 0);
                 float f[KCA];
 #pragma unroll
@@ -202,8 +220,16 @@ conv_rows_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const ui
         const int q = warp & 3;
         const uint32_t lane_addr = tmem + ((uint32_t)(q * 32) << 16);
         const int v = r0 + q * 32 + lane;
-        const int item = v / Lv, s = v - item * Lv;
-        const bool row_ok = item < B && s < L;
+        int item, s;
+        bool row_ok;
+        if constexpr (VL) {
+            item = vl_item_of_row(vl, PAD, v);
+            s = v - (vl.cum[item] + PAD * item);
+            row_ok = item < vl.n && s < vl.cum[item + 1] - vl.cum[item];
+        } else {
+            item = v / Lv, s = v - item * Lv;
+            row_ok = item < B && s < L;
+        }
         float *yp = y + ((size_t)(row_ok ? item : 0) * COUT + cg * N) * L + (row_ok ? s : 0);
         const float *bp = bias + cg * N;
 #pragma unroll 1
@@ -227,19 +253,26 @@ conv_rows_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const ui
     if constexpr (Cfg::CL > 1) cluster_sync();  // no CTA leaves while a peer may still multicast into its ring or barriers
 }
 
-template <class Cfg>
+// vt != nullptr: ragged launch (VL instantiation), B = vt->n items, L = the padded row stride
+template <class Cfg, bool VL = false>
 static int launch_conv_rows(const float *x, float *y, const uint8_t *wtc, const float *bias, int B, int L, int *status,
-                            cudaStream_t s) {
+                            cudaStream_t s, const VarLenTab *vt = nullptr) {
     static bool configured = false;
     if (!configured) {
-        MG_CUDA_TRY(cudaFuncSetAttribute(conv_rows_tc_kernel<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+        MG_CUDA_TRY(cudaFuncSetAttribute(conv_rows_tc_kernel<Cfg, VL>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
-    const long long vrows = (long long)B * (L + Cfg::PAD);
+    VarLenArg<VL> vl{};
+    long long vrows = (long long)B * (L + Cfg::PAD);
+    if constexpr (VL) {
+        vl = *vt;
+        vl.mul = 1;
+        vrows = (long long)vl.cum[vl.n] + (long long)Cfg::PAD * vl.n;  // no rows for the padding frames
+    }
     unsigned tiles = (unsigned)((vrows + Cfg::ROWS - 1) / Cfg::ROWS);
     tiles = (tiles + Cfg::CL - 1) / Cfg::CL * Cfg::CL;  // whole clusters (a tile past the last row converts zeros and stores nothing)
-    MG_CUDA_TRY(launch_ex(conv_rows_tc_kernel<Cfg>, dim3(tiles, Cfg::NCG), dim3(Cfg::NT), Cfg::SMEM_BYTES, s, Cfg::CL, true, x, y, wtc,
-                          bias, L, B, status));
+    MG_CUDA_TRY(launch_ex(conv_rows_tc_kernel<Cfg, VL>, dim3(tiles, Cfg::NCG), dim3(Cfg::NT), Cfg::SMEM_BYTES, s, Cfg::CL, true, x, y, wtc,
+                          bias, L, B, status, vl));
     return MG_OK;
 }
 
@@ -258,6 +291,12 @@ using Post1DgradCfg = ConvCfg<1024, 1024, 5, 32, false, 2, kPost1NG, 1>;  // the
 int launch_gen_pre_tc(const float *mel, float *y, const float *packed, int B, int T, int *status, cudaStream_t s) {
     const uint8_t *wtc = reinterpret_cast<const uint8_t *>(packed) + tc_region_start() + tc_pre_offset();
     return launch_conv_rows<PreCfg>(mel, y, wtc, packed + bias_offset(0), B, T, status, s);
+}
+
+// the same on a ragged batch: mel [vt->n][80][T], item b's first cum[b+1] - cum[b] frames (y: the same layout at 512 channels)
+int launch_gen_pre_tc_varlen(const float *mel, float *y, const float *packed, const VarLenTab &vt, int T, int *status, cudaStream_t s) {
+    const uint8_t *wtc = reinterpret_cast<const uint8_t *>(packed) + tc_region_start() + tc_pre_offset();
+    return launch_conv_rows<PreCfg, true>(mel, y, wtc, packed + bias_offset(0), vt.n, T, status, s, &vt);
 }
 
 // x [Bt][1024][L] -> y [Bt][1024][L] = lrelu(conv_post1(x))   (Discriminator.conv_post1)

@@ -127,6 +127,20 @@ static int generator_tc_chain(const float *packed, const float *mel, float *audi
     return MG_OK;
 }
 
+// The default chain on a ragged batch (vt: per-item lengths of this slice), whatever the A/B knobs above select: conv_pre -> a0,
+// up0 -> u, res0+up1 -> a1, res1 -> a2, up2 -> u, res2+up3 -> a1, res3+post -> audio -- the buffers the uniform default chain uses.
+static int generator_tc_chain_varlen(const float *packed, const float *mel, float *audio, const VarLenTab &vt, int T, float *a0,
+                                     float *a1, float *a2, float *u, int *status, cudaStream_t s) {
+    int rc;
+    if ((rc = launch_gen_pre_tc_varlen(mel, a0, packed, vt, T, status, s))) return rc;
+    if ((rc = launch_convt_tc_varlen(a0, u, packed, 0, vt, T, status, s))) return rc;
+    if ((rc = launch_resblock_tc_varlen(u, a1, packed, 20, vt, T, status, s))) return rc;
+    if ((rc = launch_resblock_tc_varlen(a1, a2, packed, 1, vt, T, status, s))) return rc;
+    if ((rc = launch_convt_tc_varlen(a2, u, packed, 2, vt, T, status, s))) return rc;
+    if ((rc = launch_resblock_tc_varlen(u, a1, packed, 22, vt, T, status, s))) return rc;
+    return launch_resblock_tc_varlen(a1, audio, packed, 4, vt, T, status, s);
+}
+
 // Side streams for batch slices (forked from / joined into the caller's stream with events: the call stays asynchronous
 // and stream-ordered for the caller).  Per host thread, like the rest of the library's state.
 constexpr int kMaxDevices = 64;
@@ -167,9 +181,23 @@ int generator_tc_slices(int B, int T) {
 // mel_host / audio_host (both or neither; pinned): the host-buffer entry point's copies, cut the same way -- each slice's
 // stream uploads its mel slice before its chain and downloads its audio slice after it, so all but the last download
 // overlap the other chains' kernels.
+//
+// lengths (host, B values in [1, T], checked by the caller): ragged batch -- the default chain with per-item lengths
+// (generator_tc_chain_varlen).  Slices are then cut by cumulative mel frames instead of item counts (the same >= 512 frames per
+// slice), and a slice with more than kVlMaxItems items runs as several launches in a row on its stream: each launch's
+// tables travel as kernel parameters (VarLenTab), which bounds their size.
 int launch_generator_tc(const float *packed, const float *mel, float *audio, int B, int T, float *ws, int *status,
-                        cudaStream_t s, cudaEvent_t *ev, const float *mel_host, float *audio_host) {
-    const int slices = ev ? 1 : generator_tc_slices(B, T);
+                        cudaStream_t s, cudaEvent_t *ev, const float *mel_host, float *audio_host, const int *lengths) {
+    long long frames = (long long)B * T;
+    if (lengths) {
+        frames = 0;
+        for (int i = 0; i < B; ++i) frames += lengths[i];
+    }
+    int slices = ev ? 1 : generator_tc_slices(B, T);
+    if (lengths && !ev) {  // the uniform rule on the frames that are really there
+        slices = SliceStreams::kMax < 4 ? SliceStreams::kMax : 4;
+        while (slices > 1 && (frames < 512ll * slices || B < slices)) --slices;
+    }
     float *base[6];
     for (int i = 0; i < 6; ++i) base[i] = ws + ws_offset(i, B, T);
     const size_t per_item[6] = {(size_t)512 * T, (size_t)256 * 8 * T, (size_t)128 * 64 * T, (size_t)64 * 128 * T, 0, (size_t)8192 * T};
@@ -186,8 +214,15 @@ int launch_generator_tc(const float *packed, const float *mel, float *audio, int
         MG_CUDA_TRY(cudaEventRecord(ss.fork, s));
     }
     int forked = 0;  // side streams that wait on `fork` so far: all of them are joined back, also on the error path
+    long long acc = 0;  // (ragged) mel frames of the items before b0
     for (int k = 0, b0 = 0; k < slices && rc == MG_OK; ++k) {
-        const int nb = B / slices + (k < B % slices);
+        int nb = B / slices + (k < B % slices);
+        if (lengths) {  // items up to the k+1-th share of the frames (at least one; the last slice takes the rest)
+            nb = 0;
+            for (long long a = acc; b0 + nb < B && (k == slices - 1 || nb == 0 || a < frames * (k + 1) / slices); ++nb) a += lengths[b0 + nb];
+            nb = nb < B - b0 - (slices - 1 - k) ? nb : B - b0 - (slices - 1 - k);  // every later slice keeps an item
+            for (int i = 0; i < nb; ++i) acc += lengths[b0 + i];
+        }
         cudaStream_t q = k == 0 ? s : ss.st[k - 1];
         auto slice = [&]() -> int {
             if (k > 0) {
@@ -198,8 +233,22 @@ int launch_generator_tc(const float *packed, const float *mel, float *audio, int
                 MG_CUDA_TRY(cudaMemcpyAsync(const_cast<float *>(mel) + b0 * mel_item, mel_host + b0 * mel_item,
                                             nb * mel_item * sizeof(float), cudaMemcpyHostToDevice, q));
             float *a[3] = {base[1] + b0 * per_item[1], base[2] + b0 * per_item[2], base[3] + b0 * per_item[3]};
-            int r = generator_tc_chain(packed, mel + b0 * mel_item, audio + b0 * audio_item, nb, T, base[0] + b0 * per_item[0], a,
+            int r = MG_OK;
+            if (lengths) {
+                static thread_local VarLenTab vt;  // (4 KB: not on the stack; copied into each launch's parameters)
+                for (int c0 = 0; c0 < nb && r == MG_OK; c0 += kVlMaxItems) {  // launches of at most kVlMaxItems items
+                    const int b = b0 + c0;
+                    vt.n = nb - c0 < kVlMaxItems ? nb - c0 : kVlMaxItems;
+                    vt.mul = 1;
+                    vt.cum[0] = 0;
+                    for (int i = 0; i < vt.n; ++i) vt.cum[i + 1] = vt.cum[i] + lengths[b + i];
+                    r = generator_tc_chain_varlen(packed, mel + b * mel_item, audio + b * audio_item, vt, T, base[0] + b * per_item[0],
+                                                  a[1] + c0 * per_item[2], a[2] + c0 * per_item[3], base[5] + b * per_item[5], status, q);
+                }
+            } else {
+                r = generator_tc_chain(packed, mel + b0 * mel_item, audio + b0 * audio_item, nb, T, base[0] + b0 * per_item[0], a,
                                        base[5] + b0 * per_item[5], status, q, ev);
+            }
             if (r) return r;
             if (audio_host)
                 MG_CUDA_TRY(cudaMemcpyAsync(audio_host + b0 * audio_item, audio + b0 * audio_item, nb * audio_item * sizeof(float),

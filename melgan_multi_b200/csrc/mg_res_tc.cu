@@ -187,10 +187,17 @@ __device__ __forceinline__ void store_x16_push(uint8_t *Xh, uint8_t *Xl, int xpi
     }
 }
 
-template <class Cfg>
+// VL (ragged batch, mg_gen_forward_varlen): grid.x runs over the linearised (item, super-tile) list vl.first[] (grid.y = 1; both
+// CTAs of a pair always belong to the same item), item b is vl.mul * (cum[b+1] - cum[b]) positions long and L_ is the row
+// stride of x / y (the padded length).  Everything below uses the item's own length where it used L: s_hi, `interior`, the
+// zero-padding masks, the tail ConvT's fix-up and conv_post's sequence end; tensor-map rows in [L, L_) are real memory and
+// are masked as they land; res3+post writes the exact-zero audio past the item's end.  Uniform launches (VL = false)
+// compile to the code without it.
+template <class Cfg, bool VL = false>
 __global__ void __launch_bounds__(Cfg::NT, Cfg::MINB)
-resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float *__restrict__ packed, int stage, int L, int nB,
-                   int *__restrict__ status, long long *__restrict__ trace, const __grid_constant__ CUtensorMap xmap) {
+resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float *__restrict__ packed, int stage, int L_, int nB,
+                   int *__restrict__ status, long long *__restrict__ trace, const __grid_constant__ CUtensorMap xmap,
+                   const __grid_constant__ VarLenArg<VL> vl) {
     constexpr int C = Cfg::C, NBLK = Cfg::NBLK, P = Cfg::P, SLACK = Cfg::SLACK, HALO = Cfg::HALO;
     constexpr int XPITCH = Cfg::XPITCH, XBYTES = Cfg::XBYTES, KC = Cfg::KC, CHUNK = Cfg::CHUNK, NSTAGE = Cfg::NSTAGE;
     constexpr int NEPI = Cfg::NEPI, NWG = Cfg::NWG, PARTS = Cfg::PARTS, CW = Cfg::CW, ITEMS = Cfg::ITEMS, NIW = Cfg::NIW;
@@ -225,10 +232,18 @@ resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const flo
     if constexpr (G2) {
         // cta_group::2 pairs are formed over the linearised (item, tile) list (grid.y = 1), so that only an odd TOTAL leaves one
         // phantom tile: it sits past the last tile of the last item, reads zeros (or rows it ignores) and stores nothing
-        const int nt = 1 + (L > PS ? (L - PS + PVS - 1) / PVS : 0), id = (int)blockIdx.x;
+        const int nt = 1 + (L_ > PS ? (L_ - PS + PVS - 1) / PVS : 0), id = (int)blockIdx.x;
         b = id / nt;
         stile = id - b * nt;
         if (b >= nB) { b = nB - 1; stile = nt; phantom = true; }
+    }
+    int L = L_;         // length of item b
+    const int LS = L_;  // row stride of x and y (positions per channel)
+    if constexpr (VL) {
+        static_assert(!G2 && !Cfg::UPF, "ragged launches: default-chain kernels only");
+        b = vl_item_of_tile(vl, stile);
+        stile -= vl.first[b];
+        L = vl.mul * (vl.cum[b + 1] - vl.cum[b]);
     }
     const int os = stile == 0 ? 0 : (PS - HALO) + (stile - 1) * PVS - HL;  // position of super-tile row 0
     const int o = os + rank * P;                                            // position of tile-local p = 0
@@ -728,6 +743,12 @@ resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const flo
                     w[e] = __float_as_uint(slab[(8 * j + e) * P + p]);
                     f[e] = lrelu(__uint_as_float(w[e]));
                 }
+                if constexpr (VL) {  // the map spans the padded stride: rows past the item's end are memory, not zero fill
+                    if (o + p >= L) {
+#pragma unroll
+                        for (int e = 0; e < 8; ++e) { w[e] = 0u; f[e] = 0.f; }
+                    }
+                }
                 tmem_st8(lane_addr + blk * 2 * C + c0, w);
                 uint32_t h[4], l[4];
 #pragma unroll
@@ -769,13 +790,13 @@ resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const flo
             const bool push = CL > 1 && (rank == 0 ? p >= P - Cfg::BND : p < Cfg::BND);
             const int prow = (rank == 0 ? p - (P - Cfg::BND) : SLACK + P + p) * 16;  // row offset in the peer's X buffer
             nb0 += push;
-            const float *xp = x + (size_t)b * C * L + (inr ? t : 0);
+            const float *xp = x + (size_t)b * C * LS + (inr ? t : 0);
             // all CW loads of the item are issued before the first use: one memory round trip, not CW/16
             uint32_t v[CW];
 #pragma unroll
             for (int j = 0; j < CW; ++j) {
                 const int col = (j / CH) * (C / NH) + part * CH + j % CH;
-                v[j] = inr ? __float_as_uint(__ldg(xp + (size_t)col * L)) : 0u;
+                v[j] = inr ? __float_as_uint(__ldg(xp + (size_t)col * LS)) : 0u;
             }
 #pragma unroll
             for (int c0 = 0; c0 < CW; c0 += 16) {
@@ -917,13 +938,17 @@ resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const flo
                         const int pp = p + k - 3;  // outside the tile only where it is outside the sequence too (zero padding)
                         if (pp >= 0 && pp < P) acc += Q[k * P + pp];
                     }
-                    y[(size_t)b * L + t] = tanhf(acc);
+                    y[(size_t)b * LS + t] = tanhf(acc);
                 }
+            }
+            if constexpr (VL) {  // audio past the item's end is exactly zero (written by the item's last tile)
+                if (os + PS >= L)
+                    for (int t = L + tid; t < LS; t += NEPI) y[(size_t)b * LS + t] = 0.f;
             }
         } else if constexpr (Cfg::UPT != 0) {
             // ---- tail ConvT epilogue: the thread of input position s stores the S outputs [S s - pad, S s - pad + S) of its channels
             constexpr int S = Cfg::UPT, TNG = Cfg::TNG, PADT = S / 2, COT = C / 2;
-            const int Lout = S * L;
+            const int Lout = S * LS;  // row stride of y
             const float *tbias = packed + bias_offset(1 + stage + 1);
             // ---- fix-up (first: it only needs b1s[], so it runs while the tensor core works on the ConvT): out[co][S L - pad + j] = bias + sum_ci lrelu(x[ci][L-1]) * W[ci][co][j + S], j < pad (the outputs position
             // L would own: x[L] = 0 leaves only the x[L-1] tap), by the CTA whose owned rows include position L - 1.  fp32 FFMA
@@ -1021,7 +1046,7 @@ resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const flo
             const int blk = it / PARTS, cbeg = (it % PARTS) * CW;
             const int p = blk * 128 + row, t = o + p;
             const bool valid = (p >= p_lo && p < p_hi && t < L);
-            float *yp = y + (size_t)b * C * L + (valid ? t : 0);
+            float *yp = y + (size_t)b * C * LS + (valid ? t : 0);
 #pragma unroll 1
             for (int c0 = cbeg; c0 < cbeg + CW; c0 += 32) {
                 uint32_t v[32];
@@ -1029,7 +1054,7 @@ resblock_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const flo
                 tmem_ld_wait();
                 if (valid) {
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) yp[(size_t)(c0 + j) * L] = __uint_as_float(v[j]) + pend[c0 + j];
+                    for (int j = 0; j < 32; ++j) yp[(size_t)(c0 + j) * LS] = __uint_as_float(v[j]) + pend[c0 + j];
                 }
             }
         }
@@ -1081,12 +1106,13 @@ static int make_input_map(CUtensorMap *m, const float *x, int B, int C, int L, i
     return MG_OK;
 }
 
-template <class Cfg>
+// vt != nullptr: ragged launch (VL instantiation), vt->n items, L = the padded row stride = mul * T
+template <class Cfg, bool VL = false>
 static int launch_resblock(const float *x, float *y, const float *packed, int stage, int B, int L, int *status,
-                           long long *trace, cudaStream_t s) {
+                           long long *trace, cudaStream_t s, const VarLenTab *vt = nullptr, int mul = 1) {
     static bool configured = false;
     if (!configured) {
-        MG_CUDA_TRY(cudaFuncSetAttribute(resblock_tc_kernel<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+        MG_CUDA_TRY(cudaFuncSetAttribute(resblock_tc_kernel<Cfg, VL>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
     constexpr int PS = Cfg::CL * Cfg::P, PVS = PS - Cfg::HALO - Cfg::HL;  // edge-aware tiling in super-tiles of CL tiles, see the kernel
@@ -1099,9 +1125,22 @@ static int launch_resblock(const float *x, float *y, const float *packed, int st
         if (rc) return rc;
     }
     // (G2: the (item, tile) list pairs up along x; an odd total gets one phantom tile, see the kernel)
-    const dim3 grid = Cfg::G2 ? dim3((unsigned)(((long long)ntiles * B + 1) / 2 * 2), 1) : dim3(ntiles * Cfg::CL, B);
-    MG_CUDA_TRY(launch_ex(resblock_tc_kernel<Cfg>, grid, dim3(Cfg::NT), Cfg::SMEM_BYTES, s, Cfg::CLUSTER, true, x, y,
-                          packed, stage, L, B, status, trace, xmap));
+    dim3 grid = Cfg::G2 ? dim3((unsigned)(((long long)ntiles * B + 1) / 2 * 2), 1) : dim3(ntiles * Cfg::CL, B);
+    VarLenArg<VL> vl{};
+    if constexpr (VL) {  // the (item, super-tile) list: each item gets exactly the tiles a launch of its own length would
+        vl = *vt;
+        vl.mul = mul;
+        int acc = 0;
+        for (int i = 0; i < vl.n; ++i) {
+            const int Li = mul * (vl.cum[i + 1] - vl.cum[i]);
+            vl.first[i] = acc;
+            acc += 1 + (Li > PS ? (Li - PS + PVS - 1) / PVS : 0);
+        }
+        vl.first[vl.n] = acc;
+        grid = dim3((unsigned)acc * Cfg::CL, 1);
+    }
+    MG_CUDA_TRY(launch_ex(resblock_tc_kernel<Cfg, VL>, grid, dim3(Cfg::NT), Cfg::SMEM_BYTES, s, Cfg::CLUSTER, true, x, y,
+                          packed, stage, L, B, status, trace, xmap, vl));
     return MG_OK;
 }
 
@@ -1173,6 +1212,34 @@ int launch_resblock_tc(const float *x, float *y, const float *packed, int stage,
         case 14: return launch_resblock<RbCfg<32, 4, 4, 2, 2, true, true>>(x, y, packed, 3, B, L, status, trace, s);
     }
     return set_error(MG_ERR_INVALID_ARGUMENT, "launch_resblock_tc: stage %d", stage);
+}
+
+// The default chain's four ResBlock kernels on a ragged batch: code 20 (res0+up1), 1 (res1), 22 (res2+up3), 4 (res3+post), the
+// configurations launch_resblock_tc picks for a uniform batch.  x [vt.n][C][mul T] with mul = 8 / 64 / 128 / 256, item b's first
+// mul * (cum[b+1] - cum[b]) positions.  Stage 0 runs CTA pairs if the LONGEST item would (a pair is bit-identical to the single
+// tile on a short item: the same products in the same K order; the second CTA just owns positions past the item's end).
+int launch_resblock_tc_varlen(const float *x, float *y, const float *packed, int code, const VarLenTab &vt, int T, int *status,
+                              cudaStream_t s) {
+    int maxlen = 0;
+    for (int i = 0; i < vt.n; ++i) maxlen = vt.cum[i + 1] - vt.cum[i] > maxlen ? vt.cum[i + 1] - vt.cum[i] : maxlen;
+    const int mul = code == 20 ? 8 : code == 1 ? 64 : code == 22 ? 128 : 256, LS = mul * T;
+    const bool tma = tma_input_ok(x, LS);
+    switch (code) {
+        case 20:
+            if (8 * maxlen > 128)
+                return tma ? launch_resblock<RbCfg<256, 1, 4, 4, 1, false, false, 2, 8, true>, true>(x, y, packed, 0, vt.n, LS, status, nullptr, s, &vt, mul)
+                           : launch_resblock<RbCfg<256, 1, 4, 4, 1, false, false, 2, 8>, true>(x, y, packed, 0, vt.n, LS, status, nullptr, s, &vt, mul);
+            return tma ? launch_resblock<RbCfg<256, 1, 4, 4, 1, false, false, 1, 8, true>, true>(x, y, packed, 0, vt.n, LS, status, nullptr, s, &vt, mul)
+                       : launch_resblock<RbCfg<256, 1, 4, 4, 1, false, false, 1, 8>, true>(x, y, packed, 0, vt.n, LS, status, nullptr, s, &vt, mul);
+        case 1:
+            return tma ? launch_resblock<RbCfg<128, 2, 4, 4, 1, false, false, 1, 0, true>, true>(x, y, packed, 1, vt.n, LS, status, nullptr, s, &vt, mul)
+                       : launch_resblock<RbCfg<128, 2, 4, 4, 1>, true>(x, y, packed, 1, vt.n, LS, status, nullptr, s, &vt, mul);
+        case 22:
+            return tma ? launch_resblock<RbCfg<64, 2, 2, 2, 2, false, false, 1, 2, true>, true>(x, y, packed, 2, vt.n, LS, status, nullptr, s, &vt, mul)
+                       : launch_resblock<RbCfg<64, 2, 2, 2, 2, false, false, 1, 2>, true>(x, y, packed, 2, vt.n, LS, status, nullptr, s, &vt, mul);
+        case 4: return launch_resblock<RbCfg<32, 4, 4, 2, 2, true>, true>(x, y, packed, 3, vt.n, LS, status, nullptr, s, &vt, mul);
+    }
+    return set_error(MG_ERR_INVALID_ARGUMENT, "launch_resblock_tc_varlen: code %d is not a default-chain ResBlock kernel", code);
 }
 
 // the configuration launch_resblock_tc picks for (stage code, L) with a 16-byte aligned input: evidence files (ncu captures) record

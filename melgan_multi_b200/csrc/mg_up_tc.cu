@@ -61,10 +61,13 @@ struct UpCfg {
     static_assert(CIN % KCA == 0, "A slot");
 };
 
-template <class Cfg>
+// VL (ragged batch, mg_gen_forward_varlen): item b's rows start at vl.mul * vl.cum[b] + b and it has vl.mul * (cum[b+1] - cum[b])
+// input positions; Lin is then the row stride of x (the padded length) and S * Lin that of y.  Uniform launches (VL = false)
+// compile to the code without it.
+template <class Cfg, bool VL = false>
 __global__ void __launch_bounds__(Cfg::NT, Cfg::MINB)
 convt_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float *__restrict__ packed, int Lin, int B,
-                int *__restrict__ status) {
+                int *__restrict__ status, const __grid_constant__ VarLenArg<VL> vl) {
     constexpr int CIN = Cfg::CIN, COUT = Cfg::COUT, S = Cfg::S, PAD = Cfg::PAD, NG = Cfg::NG, NB = Cfg::NB, N = Cfg::N;
     constexpr int ROWS = Cfg::ROWS, APITCH = Cfg::APITCH, ASLOT = Cfg::ASLOT, BSLOT = Cfg::BSLOT, KCA = Cfg::KCA;
     constexpr int NSA = Cfg::NSA, NSB = Cfg::NSB, NCHUNK = Cfg::NCHUNK, NCONV = Cfg::NCONV, NWG = Cfg::NWG, NIW = Cfg::NIW;
@@ -155,8 +158,16 @@ convt_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float 
 #pragma unroll 1
             for (int i = tid; i <= ROWS; i += NCONV) {
                 const int v = r0 - 1 + i;
-                const int item = v >= 0 ? v / Lv : 0, s = v - item * Lv;
-                const bool inr = (v >= 0 && item < B && s < Lin);
+                int item, s;
+                bool inr;
+                if constexpr (VL) {
+                    item = v >= 0 ? vl_item_of_row(vl, 1, v) : 0;
+                    s = v - (vl.mul * vl.cum[item] + item);
+                    inr = v >= 0 && item < vl.n && s < vl.mul * (vl.cum[item + 1] - vl.cum[item]);
+                } else {
+                    item = v >= 0 ? v / Lv : 0, s = v - item * Lv;
+                    inr = (v >= 0 && item < B && s < Lin);
+                }
                 const float *xp = x + ((size_t)(inr ? item : 0) * CIN + ca * KCA) * Lin + (inr ? s : 0);
                 float f[KCA];
 #pragma unroll
@@ -183,12 +194,21 @@ convt_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float 
         const float *bias = packed + bias_offset(1 + Cfg::STAGE) + cg * NG;
         for (int blk = wg; blk < NB; blk += NWG) {
             const int v = r0 + blk * 128 + q * 32 + lane;
-            const int item = v / Lv, s = v - item * Lv;
-            const bool row_ok = item < B;
+            int item, s, Li = Lin;  // Li: this item's input length
+            bool row_ok;
+            if constexpr (VL) {
+                item = vl_item_of_row(vl, 1, v);
+                s = v - (vl.mul * vl.cum[item] + item);
+                row_ok = item < vl.n;
+                if (row_ok) Li = vl.mul * (vl.cum[item + 1] - vl.cum[item]);
+            } else {
+                item = v / Lv, s = v - item * Lv;
+                row_ok = item < B;
+            }
             const int t0 = S * s - PAD;  // first output sample owned by this input position
             float *yb = y + ((size_t)(row_ok ? item : 0) * COUT + cg * NG) * Lout;
             if (S == 8) {
-                const bool lo_ok = row_ok && s >= 1, hi_ok = row_ok && s <= Lin - 1;
+                const bool lo_ok = row_ok && s >= 1, hi_ok = row_ok && s <= Li - 1;
 #pragma unroll 1
                 for (int j0 = 0; j0 < NG; j0 += 8) {
                     uint32_t w[8][8];
@@ -208,7 +228,7 @@ convt_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float 
                     }
                 }
             } else {  // S == 2: t0 = 2s - 1
-                const bool lo_ok = row_ok && s >= 1, hi_ok = row_ok && s <= Lin - 1;
+                const bool lo_ok = row_ok && s >= 1, hi_ok = row_ok && s <= Li - 1;
 #pragma unroll 1
                 for (int j0 = 0; j0 < NG; j0 += 16) {
                     uint32_t v0[16], v1[16];
@@ -231,16 +251,24 @@ convt_tc_kernel(const float *__restrict__ x, float *__restrict__ y, const float 
     if (warp == 0) tmem_dealloc(tmem, Cfg::TCOLS);
 }
 
-template <class Cfg>
-static int launch_convt(const float *x, float *y, const float *packed, int B, int Lin, int *status, cudaStream_t s) {
+// vt != nullptr: ragged launch (VL instantiation), vt->n items, Lin = the padded input row stride = mul * T
+template <class Cfg, bool VL = false>
+static int launch_convt(const float *x, float *y, const float *packed, int B, int Lin, int *status, cudaStream_t s,
+                        const VarLenTab *vt = nullptr, int mul = 1) {
     static bool configured = false;
     if (!configured) {
-        MG_CUDA_TRY(cudaFuncSetAttribute(convt_tc_kernel<Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+        MG_CUDA_TRY(cudaFuncSetAttribute(convt_tc_kernel<Cfg, VL>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
-    const long long vrows = (long long)B * (Lin + 1);  // Lin + 1 rows per item: position s = Lin feeds the last `pad` outputs
+    VarLenArg<VL> vl{};
+    long long vrows = (long long)B * (Lin + 1);  // Lin + 1 rows per item: position s = Lin feeds the last `pad` outputs
+    if constexpr (VL) {
+        vl = *vt;
+        vl.mul = mul;
+        vrows = (long long)mul * vl.cum[vl.n] + vl.n;  // no rows for the padding positions
+    }
     dim3 grid((unsigned)((vrows + Cfg::ROWS - 1) / Cfg::ROWS), Cfg::NCG);
-    MG_CUDA_TRY(launch_ex(convt_tc_kernel<Cfg>, grid, dim3(Cfg::NT), Cfg::SMEM_BYTES, s, 1, true, x, y, packed, Lin, B, status));
+    MG_CUDA_TRY(launch_ex(convt_tc_kernel<Cfg, VL>, grid, dim3(Cfg::NT), Cfg::SMEM_BYTES, s, 1, true, x, y, packed, Lin, B, status, vl));
     return MG_OK;
 }
 
@@ -427,6 +455,17 @@ int launch_convt_tc(const float *x, float *y, const float *packed, int stage, in
         case 3: return launch_convt<UpCfg<3>>(x, y, packed, B, Lin, status, s);
     }
     return set_error(MG_ERR_INVALID_ARGUMENT, "launch_convt_tc: stage %d", stage);
+}
+
+// The same on a ragged batch (the default chain's two stand-alone ConvTs, stages 0 and 2): x [vt.n][Cin][mul T], item b's
+// first mul * (cum[b+1] - cum[b]) positions; y [vt.n][Cout][S mul T], the first S times as many.
+int launch_convt_tc_varlen(const float *x, float *y, const float *packed, int stage, const VarLenTab &vt, int T, int *status,
+                           cudaStream_t s) {
+    switch (stage) {
+        case 0: return launch_convt<UpCfg<0>, true>(x, y, packed, vt.n, T, status, s, &vt, 1);
+        case 2: return launch_convt<UpCfg<2>, true>(x, y, packed, vt.n, 64 * T, status, s, &vt, 64);
+    }
+    return set_error(MG_ERR_INVALID_ARGUMENT, "launch_convt_tc_varlen: stage %d has no ragged form", stage);
 }
 
 }  // namespace mg

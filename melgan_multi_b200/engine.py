@@ -42,6 +42,9 @@ def lib():
         L.mg_gen_forward.restype = ctypes.c_int
         L.mg_gen_forward.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
                                      ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
+        L.mg_gen_forward_varlen.restype = ctypes.c_int
+        L.mg_gen_forward_varlen.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
         L.mg_gen_forward_timed.restype = ctypes.c_int
         L.mg_gen_forward_timed.argtypes = L.mg_gen_forward.argtypes + [ctypes.POINTER(ctypes.c_float)]
         L.mg_gen_check_status.restype = ctypes.c_int
@@ -131,6 +134,9 @@ def lib():
         L.mg_gen_engine_forward.restype = ctypes.c_int
         L.mg_gen_engine_forward.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
                                             ctypes.c_int]
+        L.mg_gen_engine_forward_varlen.restype = ctypes.c_int
+        L.mg_gen_engine_forward_varlen.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+                                                   ctypes.c_int, ctypes.c_void_p]
         L.mg_gen_engine_last_kernel_ms.restype = ctypes.c_int
         L.mg_gen_engine_last_kernel_ms.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_float)]
         L.mg_gen_engine_destroy.restype = None
@@ -146,6 +152,23 @@ def check(rc):
 
 def _ptr_array(ptrs):
     return (ctypes.c_void_p * len(ptrs))(*ptrs)
+
+
+def lengths_array(lengths, B):
+    """Per-item mel lengths (list, tuple, numpy array or integer torch tensor; a CUDA tensor is copied to the host, which
+    synchronises with its stream) as the host int32 array the ragged entry points take.  Range checks are the library's."""
+    if hasattr(lengths, "detach"):  # torch tensor
+        if lengths.is_floating_point() or lengths.is_complex():
+            raise EngineError("lengths must be integers, got %s" % (lengths.dtype,))
+        lengths = lengths.detach().cpu().numpy()
+    a = np.asarray(lengths)
+    if a.ndim != 1 or a.shape[0] != B:
+        raise EngineError("lengths must hold one value per batch item (%d), got shape %s" % (B, a.shape))
+    if a.size and not np.issubdtype(a.dtype, np.integer):
+        raise EngineError("lengths must be integers, got %s" % (a.dtype,))
+    if a.size and (a.min() < np.iinfo(np.int32).min or a.max() > np.iinfo(np.int32).max):
+        raise EngineError("lengths out of the int32 range")
+    return (ctypes.c_int * B)(*a.astype(np.int64).tolist())
 
 
 class _StatusWatch:
@@ -243,7 +266,10 @@ class GeneratorDevice:
             self._ws = self.torch.empty((need + 3) // 4, dtype=self.torch.float32, device=self.device)
         return self._ws
 
-    def forward(self, mel, out=None):
+    def forward(self, mel, out=None, lengths=None):
+        """mel [B, 80, T] -> audio [B, 1, 256 T], asynchronous on the current stream.  lengths (optional, one value in [1, T]
+        per item; see lengths_array): ragged batch -- item b is its first lengths[b] frames, its audio ends at 256 lengths[b]
+        samples and is exactly zero after that (mg_gen_forward_varlen)."""
         torch = self.torch
         if mel.dim() != 3 or mel.shape[1] != 80:
             raise EngineError("mel must be [B, 80, T], got %s" % (tuple(mel.shape),))
@@ -251,14 +277,19 @@ class GeneratorDevice:
             raise EngineError("mel must be an fp32 tensor on %s" % (self.device,))
         mel = mel.contiguous()
         B, _, T = mel.shape
+        lens = None if lengths is None else lengths_array(lengths, B)
         if out is None:
             out = torch.empty((B, 1, 256 * T), dtype=torch.float32, device=self.device)
         self._watch.check()  # the previous forward's status word, if its copy has landed
         ws = self.workspace(B, T)
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream().cuda_stream
-            check(lib().mg_gen_forward(self.packed.data_ptr(), mel.data_ptr(), out.data_ptr(), B, T,
-                                       ws.data_ptr(), ws.numel() * 4, stream))
+            if lens is None:
+                check(lib().mg_gen_forward(self.packed.data_ptr(), mel.data_ptr(), out.data_ptr(), B, T,
+                                           ws.data_ptr(), ws.numel() * 4, stream))
+            else:
+                check(lib().mg_gen_forward_varlen(self.packed.data_ptr(), mel.data_ptr(), out.data_ptr(), B, T, lens,
+                                                  ws.data_ptr(), ws.numel() * 4, stream))
             off = (lib().mg_gen_workspace_bytes(B, T) - 256) // 4  # the status word sits after the activation buffers
             self._watch.arm(ws.view(torch.int32)[off:off + 1])
         return out
@@ -662,14 +693,18 @@ class GeneratorHost:
                 lst.append(a.ctypes.data)
         check(lib().mg_gen_engine_load_state(self._h, _ptr_array(vs), _ptr_array(gs), _ptr_array(bs)))
 
-    def forward(self, mel, out=None):
+    def forward(self, mel, out=None, lengths=None):
+        """lengths (optional, one value in [1, T] per item): ragged batch, as GeneratorDevice.forward."""
         mel = np.ascontiguousarray(mel, dtype=np.float32)
         B, C, T = mel.shape
         if C != 80:
             raise EngineError("mel must be [B, 80, T]")
         if out is None:
             out = np.empty((B, 1, 256 * T), np.float32)
-        check(lib().mg_gen_engine_forward(self._h, mel.ctypes.data, out.ctypes.data, B, T))
+        if lengths is None:
+            check(lib().mg_gen_engine_forward(self._h, mel.ctypes.data, out.ctypes.data, B, T))
+        else:
+            check(lib().mg_gen_engine_forward_varlen(self._h, mel.ctypes.data, out.ctypes.data, B, T, lengths_array(lengths, B)))
         return out
 
     def forward_ptr(self, mel_ptr, out_ptr, B, T):

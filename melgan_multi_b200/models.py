@@ -178,13 +178,22 @@ class Generator(nn.Module):
                 x = F.conv1d(F.leaky_relu(h), ws[b], bs[b], padding=1) + x
         return torch.tanh(F.conv1d(F.leaky_relu(x), ws[29], bs[29], padding=3))
 
-    def forward(self, x):
+    def forward(self, x, lengths=None):
+        """lengths (optional): ragged batch -- one mel length in [1, T] per item (list, tuple or integer tensor; a CUDA
+        tensor costs one host synchronisation to read).  Item b is then x[b, :, :lengths[b]]; its audio fills the first
+        256 * lengths[b] samples, bit-identical to a forward of that item alone, and is exactly 0 after them.  Inference
+        only: a call that would need autograd raises EngineError (training uses fixed-length segments)."""
         if not x.is_cuda:
             raise _engine.EngineError("melgan_multi_b200.Generator.forward needs a CUDA tensor (no CPU fallback)")
         if x.dtype != torch.float32:
             x = x.float()
         vs, gs, bs = self._param_triplets()
         needs_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in vs + gs + bs))
+        if lengths is not None:
+            if needs_grad:
+                raise _engine.EngineError("Generator.forward(x, lengths): ragged batches are inference-only; call it under "
+                                          "torch.no_grad() / torch.inference_mode() or with parameters that need no grad")
+            return self._ensure_packed().forward(x, lengths=lengths)
         if not needs_grad:
             return self._engine_forward(x)
         flat = []
